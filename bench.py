@@ -31,6 +31,17 @@ ratio): the oracle runs the real interior-point iterations and the KKT sections 
 iterations are timed.  When a single step costs more than the time budget allows (C5: ~2.5 min
 per factorisation), the one step that is timed is the solver's own first factorisation
 (solver_default_start!, identity scaling) + 3 solves; `steps` in the line says how many were timed.
+
+--dump-outputs DIR : after the timed steps, writes what the last timed step computed, as its caller
+reads it back: solve<k>_x.npy and solve<k>_z.npy (lhsx / lhsz of the step's k-th solve), float64,
+at most 64 MB in all (a longer array is replaced by a fixed, seeded sample of its entries).
+--replay-inputs PATH : the replayed systems are iterates of this build's own GPU solve, so they
+depend on the build (a different summation order moves the trajectory, even the iteration count)
+and, for C2, on the run (FP64 atomics in its root-front assembly).  With --replay-inputs the first
+run stores its replayed systems (cone states and right-hand sides) in PATH and every later run with
+the same PATH replays those instead: runs with the same arguments then solve the same systems, on any
+build, and their dumps can be compared output for output.  C2's outputs can still differ in the last
+bits from run to run (the same atomics, in the timed factorisations).
 """
 import argparse
 import json
@@ -297,6 +308,72 @@ def reference_arm(name, steps, warmup):
     return line
 
 
+DUMP_BUDGET_BYTES = 64_000_000
+
+
+def fit_dump_budget(outs, budget=DUMP_BUDGET_BYTES):
+    """float64 copies of `outs` that together stay within `budget` bytes: an array longer than its
+    equal share is replaced by a fixed sample of its entries (seed 0, ascending indices), so the
+    same array sizes always give the same sample."""
+    cap = (budget - 4096 * len(outs)) // (8 * len(outs))      # 4 KB per file for the .npy header
+    fitted = {}
+    for name, a in outs.items():
+        a = np.asarray(a, dtype=np.float64)
+        if a.size > cap:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        fitted[name] = a
+    return fitted
+
+
+def dump_outputs(out_dir, ks, rhs_t, write):
+    """The solutions of the last timed step (device-resident leg).  The step leaves only its last
+    solution on the device; the earlier ones are solved again from the same factorisation and
+    right-hand sides (a solve reads the factorisation, it does not change it).  Every rank takes part
+    in the solves; only `write` ranks write."""
+    N, n, m = ks.KKT.shape[0], ks.n, ks.m
+    sols = [None] * len(rhs_t)
+    sols[-1] = ks.ldl.download(6, N)
+    for k, (tx, tz) in enumerate(rhs_t[:-1]):
+        ks.setrhs_staged(tx.data_ptr() if tx.numel() else 0, tz.data_ptr() if tz.numel() else 0)
+        ks.solve(None, None)
+        sols[k] = ks.ldl.download(6, N)
+    if not write:
+        return
+    outs = {}
+    for k, x in enumerate(sols, 1):
+        outs[f"solve{k}_x"], outs[f"solve{k}_z"] = x[:n], x[n:n + m]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in fit_dump_budget(outs).items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def save_replay(path, name, n, m, replay_ids, replay):
+    arrs = dict(workload=np.array(name), n_m=np.array([n, m]), replay_ids=np.array(replay_ids))
+    for i, s_ in enumerate(replay):
+        for k, v in s_["state"].items():
+            arrs[f"s{i}_state_{k}"] = v
+        for j, (rx, rz) in enumerate(s_["rhs"]):
+            arrs[f"s{i}_rx{j}"], arrs[f"s{i}_rz{j}"] = rx, rz
+    with open(path, "wb") as f:
+        np.savez(f, **arrs)
+
+
+def load_replay(path, name, n, m):
+    """(replay_ids, replay) as save_replay stored them; the file must hold systems of this instance."""
+    with np.load(path) as z:
+        if str(z["workload"]) != name or z["n_m"].tolist() != [n, m]:
+            raise SystemExit(f"{path} holds systems of {z['workload']} (n, m = {z['n_m'].tolist()}), "
+                             f"not of {name} (n, m = {[n, m]})")
+        ids = z["replay_ids"].tolist()
+        replay = []
+        for i in range(len(ids)):
+            pre = f"s{i}_state_"
+            st = {f[len(pre):]: z[f] for f in z.files if f.startswith(pre)}
+            nrhs = sum(f.startswith(f"s{i}_rx") for f in z.files)
+            replay.append(dict(state=st, rhs=[(z[f"s{i}_rx{j}"], z[f"s{i}_rz{j}"]) for j in range(nrhs)]))
+    return ids, replay
+
+
 def _watchdog(seconds):
     """A hung collective must not hang the caller: dump stacks and exit non-zero."""
     import faulthandler
@@ -321,7 +398,15 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default=os.environ.get("CB200_WORKLOAD", "C5"))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the solutions of the last timed step to DIR/<name>.npy")
+    ap.add_argument("--replay-inputs", metavar="PATH",
+                    help="replay the systems stored in PATH; if PATH does not exist, store this run's there")
     args = ap.parse_args()
+    if (args.dump_outputs or args.replay_inputs) and args.impl == "reference":
+        ap.error("--dump-outputs and --replay-inputs apply to --impl b200")
+    # decided before any rank can have written PATH
+    load_inputs = bool(args.replay_inputs) and os.path.exists(args.replay_inputs)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -360,6 +445,10 @@ def main():
     rec.steps = None
     n, m = solver.data.n, solver.data.m
     N = ks.KKT.shape[0]
+    if load_inputs:
+        replay_ids, replay = load_replay(args.replay_inputs, name, n, m)
+    elif args.replay_inputs and rank == 0:
+        save_replay(args.replay_inputs, name, n, m, replay_ids, replay)
 
     def pinned(a):
         """copy of `a` in page-locked host memory (the e2e copies are then true DMA transfers)"""
@@ -440,6 +529,8 @@ def main():
     tm = ks.ldl.timers()
     ir_per_solve = ks.ir_rounds / max(1, ks.n_solves)
     stop.set(); th.join(timeout=2)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ks, staged[(args.warmup + args.steps - 1) % len(replay)][1], rank == 0)
     ks.ldl.set_resident(False)
     # ---- per-kernel-class timing of the factorisation (events around each launch group; graph
     # replay is off for these extra steps, they are not part of the timed regions above).  In
